@@ -26,8 +26,18 @@ output.  A "step" is one LDE of one synthetic matrix (uniform field elements, se
               independent commitment per shard + one all-gather of roots).  Every rank asserts cap == the N=1 cap.
   others      (N=1 only) the remaining single-GPU BASELINE configs timed the same way.
 
+--steps K times exactly K steps of the primary workload (`value`, `ms_per_step`, `roofline`); its warm-up is max(--warmup, 3)
+steps.  The other legs use their own counts: e2e min(max(K, 4), 10) calls, --impl reference min(K, 5) steps, and the secondary
+workloads and sharded_commit fixed counts sized to their run time.
+
 --impl reference: times the reference's CPU algorithm (the oracle port — the reference is Rust and cannot be built in this
 image) on the same metric with all physical cores; rank 0 only under torchrun.
+
+--dump-outputs DIR: after the timed steps of the primary workload, writes what its last step computed (the LDE output, raw
+Montgomery words as float64, which holds them exactly) for a fixed, seeded sample of DUMP_ROWS rows, as DIR/coset_lde.npy, and
+the sampled row indices as DIR/coset_lde_rows.npy.  Inputs are seeded, so two builds run with the same arguments can be compared
+file for file.  Under torchrun rank r writes DUMP_ROWS / N^2 rows of its own row block (each row 100N columns wide) as
+coset_lde_rank<r>.npy, so the N ranks together write as many elements as one GPU does.
 """
 import argparse
 import json
@@ -46,6 +56,7 @@ ALG_BYTES = ((1 << LOG_H) * W + (1 << (LOG_H + ADDED_BITS)) * W) * 4       # 1,2
 OUT_ELEMS = (1 << (LOG_H + ADDED_BITS)) * W                                   # 209,715,200
 BUTTERFLIES = 3 * LOG_H * (1 << (LOG_H - 1)) * W                              # 3.146e9 (iDFT + two coset DFTs)
 T_LOG_H, T_W, T_CAP = 20, 1312, 3                                             # config 5 trace
+DUMP_ROWS = 1 << 16                   # 2^16 rows x 100 cols of float64 = 52 MB over all ranks, under the 64 MB a dump may take
 
 
 def parse():
@@ -58,7 +69,27 @@ def parse():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-sharded", action="store_true", help="skip the config-5 sharded commit")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-pointer leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the primary workload's last output to DIR/*.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return args
+
+
+def dump_outputs(out_dir, rows, name, count):
+    """Seeded sample of `count` rows of `rows` (a CUDA int32 tensor) as float64 .npy files; the sample depends only on the
+    row counts, so runs with the same arguments sample the same rows."""
+    import numpy as np
+    import torch
+    d = pathlib.Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    n = rows.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(n, size=min(n, count), replace=False))
+    sample = rows.index_select(0, torch.from_numpy(idx).to(rows.device)).cpu().numpy()
+    np.save(d / f"{name}.npy", sample.astype(np.float64))
+    np.save(d / f"{name}_rows.npy", idx.astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -159,11 +190,20 @@ def _omp_setup():
     return phys
 
 
+def _native_oracle():
+    """The oracle compiled with -march=native for THIS host (the in-tree build may come from another CPU, and an illegal
+    instruction would kill the bench), in a temporary directory: the bench writes nothing into the tree."""
+    import tempfile
+    from oracle import p3_oracle as O
+    with tempfile.TemporaryDirectory() as d:
+        O.lib(O.build(native=True, out=pathlib.Path(d) / "libp3oracle.so"))    # stays mapped after the directory is gone
+    return O
+
+
 def cpu_lde_throughput(budget_s=15.0):
     """Oracle port of coset_lde_batch on a bounded column sample of the same workload.  Returns (Gelem/s, cores, sample)."""
     cores = _omp_setup()
-    from oracle import p3_oracle as O
-    O.build(native=True)          # rebuild with -march=native for THIS host
+    O = _native_oracle()
     f = 1
     m = O.random_matrix(f, 1 << LOG_H, 4, seed=1)
     t0 = time.time(); O.coset_lde_batch(f, m, ADDED_BITS, O.generator(f)); t4 = time.time() - t0
@@ -195,8 +235,7 @@ def run_reference(args):
     if rank != 0:
         return
     cores = _omp_setup()
-    from oracle import p3_oracle as O
-    O.build(native=True)
+    O = _native_oracle()
     f = 1
     cols = W if cores >= 16 else 16          # full workload on a many-core host, a 16-column sample on small hosts
     m = O.random_matrix(f, 1 << LOG_H, cols, seed=1)
@@ -305,6 +344,11 @@ def main():
     with ClockSampler(local) as clk:
         ms, launches = timed(lde_step, args.steps, warm)
     value = world * OUT_ELEMS / (ms * 1e-3) / 1e9
+    if args.dump_outputs:
+        if world == 1:
+            dump_outputs(args.dump_outputs, out, "coset_lde", DUMP_ROWS)
+        else:
+            dump_outputs(args.dump_outputs, grp.rows_tensor(), f"coset_lde_rank{rank}", DUMP_ROWS // (world * world))
 
     line = {
         "metric": "coset_lde_batch output Gelem/s (KoalaBear 2^20 x 100 per GPU, blowup 2)", "value": value, "unit": "Gelem/s",

@@ -21,12 +21,12 @@ BABY_BEAR, KOALA_BEAR = 0, 1
 P2_MAXW = 24
 
 
-def build(native: bool = False) -> pathlib.Path:
-    """Compile the oracle with the system gcc (oracle/Makefile)."""
-    so = _HERE / "_build" / "libp3oracle.so"
+def build(native: bool = False, out=None) -> pathlib.Path:
+    """Compile the oracle with the system gcc (oracle/Makefile), into oracle/_build or to the path `out`."""
+    so = pathlib.Path(out).resolve() if out else _HERE / "_build" / "libp3oracle.so"
     src = _HERE / "p3_oracle.c"
     if native or not so.exists() or so.stat().st_mtime < src.stat().st_mtime:
-        subprocess.run(["make", "-C", str(_HERE), "-B" if native else "-s"], check=True,
+        subprocess.run(["make", "-C", str(_HERE), "-B" if native else "-s", f"OUT={so}"], check=True,
                        stdout=subprocess.DEVNULL)
     return so
 
@@ -49,11 +49,11 @@ class Hasher(C.Structure):
 _lib = None
 
 
-def lib():
+def lib(so=None):
+    """The loaded oracle; the first call loads `so` if given, else the in-tree build."""
     global _lib
     if _lib is None:
-        so = build()
-        L = C.CDLL(str(so))
+        L = C.CDLL(str(so or build()))
         u32, u64, sz, p32 = C.c_uint32, C.c_uint64, C.c_size_t, C.POINTER(C.c_uint32)
         for name, res, args in [
             ("p3o_prime", u32, [C.c_int]), ("p3o_add", u32, [C.c_int, u32, u32]), ("p3o_sub", u32, [C.c_int, u32, u32]),

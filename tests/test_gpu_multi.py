@@ -63,7 +63,7 @@ def _worker(rank, world, port, q):
 
 def test_sharded_commit_nccl():
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     world = 2
     ctx = mp.get_context("spawn")
     q = ctx.Queue()
