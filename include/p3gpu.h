@@ -245,8 +245,8 @@ int32_t p3gpu_merkle_paths_dev(p3gpu_ctx *ctx, const uint32_t *d_layers, const s
 /* ---- multi-GPU: one process per GPU, peer memory over NVLink (SURVEY.md 8e; DESIGN.md section 5) ------------------
  * The path shards by COLUMN for the LDE (every column is an independent polynomial, dft/src/traits.rs:22-24) and by
  * ROW RANGE for the Merkle tree (a leaf is a sequential sponge over the whole row, merkle_tree.rs:309-317; rows
- * [k*H/G, (k+1)*H/G) of the bit-reversed LDE are a complete sub-tree).  The re-sharding all-to-all is fused into the
- * LDE's last pass: its stores go straight into the destination rank's row block through CUDA-IPC-mapped peer pointers.
+ * [k*H/G, (k+1)*H/G) of the bit-reversed LDE are a complete sub-tree).  The re-sharding all-to-all copies the LDE's
+ * column chunks into the destination ranks' row blocks through CUDA-IPC-mapped peer pointers on the copy engines.
  * No collective library is involved; the host only exchanges 64-byte IPC handles once (any channel: MPI, sockets,
  * torch.distributed, ...) and fills a p3gpu_peer_group. */
 #define P3GPU_PEER_CTRL_BYTES 65536   /* size of every rank's control block (p3gpu_malloc'ed, zeroed, IPC-exported) */
@@ -273,8 +273,9 @@ int32_t p3gpu_peer_allgather_dev(p3gpu_ctx *ctx, const p3gpu_peer_group *grp, si
 
 /* coset_lde_batch of this rank's column block [col_off, col_off + w_local) of a trace of width w_total; the
  * bit-reversed-row result is scattered by row range: LDE row r goes to grp->rows[r / (H/world)] (local row r % (H/world),
- * columns col_off.., pitch w_total).  Needs w_local % 4 == 0 (column blocks that are multiples of 8 keep every 32-byte
- * store segment sector-aligned) and H / world >= 1024.  Complete on all ranks only after a following barrier. */
+ * columns col_off.., pitch w_total).  Needs w_local, w_total and col_off to be multiples of 4 (16-byte aligned rows;
+ * column blocks that are multiples of 8 keep every 32-byte row segment sector-aligned) and H / world >= 1024.  Complete on
+ * all ranks only after a following barrier. */
 int32_t p3gpu_coset_lde_batch_sharded_dev(p3gpu_ctx *ctx, int field, const p3gpu_peer_group *grp, const uint32_t *d_in, size_t h,
                                           size_t w_local, unsigned added_bits, uint32_t shift, size_t w_total, size_t col_off);
 

@@ -139,8 +139,6 @@ int32_t open_reduce(p3gpu_ctx *ctx, int field, u32 *d_ro, const u32 *d_r, const 
 int32_t ntt_coset_lde_sharded(p3gpu_ctx *ctx, int field, const u32 *d_in, size_t h, size_t w_local, unsigned added_bits, u32 shift,
                               unsigned world, u32 *const *rank_out, size_t w_total, size_t col_off, int chunk_major = 0);
 std::vector<size_t> shard_chunk_bounds(size_t w_local);
-int32_t peer_push_rows(p3gpu_ctx *ctx, cudaStream_t stream, unsigned world, u32 *const *rows, const u32 *d_src, size_t H, size_t wc, size_t w_total,
-                       size_t dst_col, unsigned log_rows);
 int32_t peer_barrier(p3gpu_ctx *ctx, unsigned world, unsigned rank, void *const *ctrl, u32 epoch, double timeout_s);
 int32_t peer_allgather(p3gpu_ctx *ctx, unsigned world, unsigned rank, void *const *tables, const u32 *d_src, size_t words);
 

@@ -1,14 +1,12 @@
 // Multi-GPU plumbing of the row-sharded commit (SURVEY.md section 8e) over NVLink peer memory, with no collective library on the
-// data path: one process per GPU, buffers shared through CUDA IPC handles (exchanged by the host over any channel), and three
-// device-side primitives on mapped peer pointers:
-//   * the LDE's last pass stores its tiles straight into the destination rank's row block (ntt.cu, PassArgs::shard_out):
-//     the all-to-all of column blocks into row blocks is fused into the transform;
+// data path: one process per GPU, buffers shared through CUDA IPC handles (exchanged by the host over any channel), and
+// primitives on mapped peer pointers:
+//   * the all-to-all of column blocks into row blocks: the LDE's column chunks are copied into the destination ranks' row
+//     blocks on the copy engines (ntt.cu, ntt_coset_lde_sharded);
 //   * peer_allgather_kernel: every rank stores a small record (a sub-tree root, a FRI final polynomial) into slot `rank` of
 //     every rank's table;
 //   * peer_barrier_kernel: flag barrier with system-scope release/acquire; stream-ordered, so "all peers' stores have landed"
 //     becomes a dependency of the next kernel on this stream without any host round trip.
-#include <algorithm>
-
 #include "common.h"
 
 namespace p3 {
@@ -27,8 +25,8 @@ __device__ __forceinline__ u32 ld_acquire_sys(const u32 *p) {
 struct PeerPtrs { u32 *p[PEER_MAX]; };
 
 // One warp.  Lane q < world: publish `epoch` in flags[rank] of rank q, then wait until flags[q] of OUR block reached `epoch`.
-// Epochs only grow (the caller passes 1, 2, 3, ...), so no reset and no ABA.  All stores of earlier kernels on this stream
-// (the LDE's peer stores) are complete before this kernel starts; the release store orders them before the flag.
+// Epochs only grow (the caller passes 1, 2, 3, ...), so no reset and no ABA.  All writes of earlier work on this stream
+// (the LDE's peer copies) are complete before this kernel starts; the release store orders them before the flag.
 __global__ void peer_barrier_kernel(const PeerPtrs ctrl, unsigned world, unsigned rank, u32 epoch, unsigned long long timeout_ns) {
     const unsigned q = threadIdx.x;
     if (q < world) {
@@ -56,34 +54,6 @@ __global__ void peer_allgather_kernel(const PeerPtrs tables, unsigned world, uns
     if (i >= words) return;
     const u32 v = src[i];
     for (unsigned q = 0; q < world; q++) tables.p[q][(size_t)rank * words + i] = v;
-}
-
-// Row-block push of the "staged" exchange: S is this rank's LDE of one column chunk (H x wc, dense); row r of S goes to rank
-// r >> log_rows, local row r & (2^log_rows - 1), columns [dst_col, dst_col + wc) of its row block (pitch w_total).  One 16-byte
-// vector per thread: consecutive lanes write consecutive 16-byte pieces of a wc*4-byte row segment, so the NVLink writes are
-// 128-byte lines instead of the 32-byte tile rows of the fused variant.
-struct PushArgs { u32 *dst[PEER_MAX]; const u32 *src; size_t n_vec, w_total, dst_col; unsigned vec_per_row, log_rows; };
-__global__ void __launch_bounds__(256) peer_push_rows_kernel(const PushArgs a) {
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < a.n_vec; i += (size_t)gridDim.x * blockDim.x) {
-        const size_t row = i / a.vec_per_row;
-        const unsigned v = (unsigned)(i - row * a.vec_per_row);
-        const uint4 x = __ldg(reinterpret_cast<const uint4 *>(a.src) + i);
-        u32 *d = a.dst[row >> a.log_rows] + (row & (((size_t)1 << a.log_rows) - 1)) * a.w_total + a.dst_col + 4u * v;
-        *reinterpret_cast<uint4 *>(d) = x;
-    }
-}
-
-int32_t peer_push_rows(p3gpu_ctx *ctx, cudaStream_t stream, unsigned world, u32 *const *rows, const u32 *d_src, size_t H, size_t wc, size_t w_total,
-                       size_t dst_col, unsigned log_rows) {
-    P3_CHECK(wc % 4 == 0 && w_total % 4 == 0 && dst_col % 4 == 0, P3GPU_EINVAL, "staged exchange needs 16-byte aligned column blocks");
-    PushArgs a;
-    for (unsigned q = 0; q < PEER_MAX; q++) a.dst[q] = q < world ? rows[q] : nullptr;
-    a.src = d_src; a.n_vec = H * (wc / 4); a.w_total = w_total; a.dst_col = dst_col; a.vec_per_row = (unsigned)(wc / 4); a.log_rows = log_rows;
-    const size_t blocks = std::min<size_t>((a.n_vec + 255) / 256, (size_t)ctx->sm_count * 4);   // a few CTAs per SM next to the NTT kernel
-    peer_push_rows_kernel<<<(unsigned)blocks, 256, 0, stream>>>(a);
-    ctx->launches++;
-    P3_CUDA(cudaGetLastError());
-    return P3GPU_OK;
 }
 
 int32_t peer_barrier(p3gpu_ctx *ctx, unsigned world, unsigned rank, void *const *ctrl, u32 epoch, double timeout_s) {

@@ -52,6 +52,18 @@ def test_product_never_imports_oracle():
             assert not pat.search(f.read_text()), f
 
 
+def test_library_has_no_variant_switches():
+    """The NTT pass kernels and the sharded LDE's exchange have one code path each: no environment variable picks a kernel
+    variant, tile shape, pass depth or exchange mode.  In particular every rank derives the same exchange chunks (and with them
+    the chunk-major row-block layout of the sharded commit) whatever its environment."""
+    removed = ["P3GPU_SHARD_MODE", "P3GPU_SHARD_CHUNK", "P3GPU_NTT_THREADS", "P3GPU_NTT_CT", "P3GPU_NTT_LOGCT", "P3GPU_NTT_MAXR",
+               "P3GPU_NTT_GENERIC", "P3GPU_NTT_TILED", "P3GPU_NTT_NOBFLY", "P3GPU_NTT_NOLOAD", "P3GPU_NTT_NOSTORE"]
+    for f in (ROOT / "plonky3_b200" / "csrc").iterdir():
+        if f.suffix in (".cu", ".cuh", ".h"):
+            found = [n for n in removed if re.search(rf"\b{n}\b", f.read_text())]
+            assert not found, (f.name, found)
+
+
 def test_field_helpers_match_reference_constants():
     # SURVEY Appendix A (baby_bear.rs:17-68, koala_bear.rs:20-94)
     assert BabyBear.ONE == 0x0FFFFFFE and KoalaBear.ONE == 0x01FFFFFE

@@ -42,7 +42,7 @@ def _worker(rank, world, port, q):
         ok = np.array_equal(cap.cpu().numpy().view(np.uint32), exp_cap)
         exp_root = O.merkle_tree(ohs, [O.coset_lde_batch(f.id, full[:, c0:c1], 1, f.generator, True)])[-1][0]
         ok2 = np.array_equal(roots[rank].cpu().numpy().view(np.uint32), exp_root)
-        # peer-memory mode (no NCCL on the data path): IPC-mapped row blocks, LDE stores fused with the re-sharding
+        # peer-memory mode (no NCCL on the data path): IPC-mapped row blocks, LDE column chunks copied into them on the copy engines
         from plonky3_b200.distributed import PeerGroup
         H = 2 << LOG_H
         grp = PeerGroup(gpu, H // world, W)

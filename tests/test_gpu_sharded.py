@@ -1,5 +1,5 @@
-"""The row-sharded multi-GPU commit (p3gpu_coset_lde_batch_sharded_dev / p3gpu_commit_sharded_dev: peer-memory stores from
-the LDE's last pass, flag barrier, peer all-gather of the cap slices) exercised on whatever the box has.
+"""The row-sharded multi-GPU commit (p3gpu_coset_lde_batch_sharded_dev / p3gpu_commit_sharded_dev: peer copies of the LDE's
+column chunks into the owners' row blocks, flag barrier, peer all-gather of the cap slices) exercised on whatever the box has.
 
   * test_sharded_lde_scatters_row_blocks: the store addressing of the sharded LDE, `world` ranks simulated inside this process
     on cuda:0 (no barrier involved);
@@ -36,13 +36,13 @@ def _gpus(n):
     return out
 
 
-@pytest.mark.parametrize("mode", ["dma", "staged", "fused"])
-@pytest.mark.parametrize("f,log_h,w,world", [(KoalaBear, 12, 100, 2), (BabyBear, 13, 72, 4), (KoalaBear, 14, 328, 8), (KoalaBear, 15, 200, 2)])
-def test_sharded_lde_scatters_row_blocks(f, log_h, w, world, mode, monkeypatch):
-    """Every rank's column-block LDE lands in the right rows/columns of every rank's row block — both exchange variants:
-    `staged` (column chunks into a staging buffer + coalesced push kernel on a second stream) and `fused` (the last pass of the
-    transform stores its tiles straight into the owners' row blocks); `dma` (default) = staged with 2-D peer copies."""
-    monkeypatch.setenv("P3GPU_SHARD_MODE", mode)
+@pytest.mark.parametrize("f,log_h,w,world", [(KoalaBear, 12, 100, 1), (BabyBear, 13, 72, 1), (KoalaBear, 11, 64, 1), (BabyBear, 10, 40, 1),
+                                             (KoalaBear, 12, 100, 2), (BabyBear, 12, 100, 2), (KoalaBear, 15, 200, 2), (BabyBear, 13, 72, 4),
+                                             (KoalaBear, 13, 72, 4), (BabyBear, 16, 264, 4), (KoalaBear, 14, 328, 8), (BabyBear, 14, 328, 8)])
+def test_sharded_lde_scatters_row_blocks(f, log_h, w, world):
+    """Every rank's column-block LDE lands in the right rows/columns of every rank's row block: column chunks are transformed
+    into a staging buffer and copied to their owners with 2-D peer copies.  A single rank stores its LDE straight into its
+    block, through the tiled pipelined transform or, for heights below 2^12, the generic network."""
     gpus = _gpus(world)
     H = 2 << log_h
     groups = PeerGroup.simulate(gpus, H // world, w)
@@ -110,7 +110,7 @@ def _rank_main(rank, world, port, q):
         q.put((rank, False, repr(e)))
 
 
-@pytest.mark.parametrize("world", [2, 4, 8])
+@pytest.mark.parametrize("world", [1, 2, 4, 8])
 def test_sharded_commit_equals_single_commit(world):
     """cap of the sharded commit (on every rank) == cap of TwoAdicFriPcs::commit on the whole trace (oracle); every rank's row
     block == its rows of the full LDE; every rank's sub-tree == its slice of the oracle's tree."""
